@@ -29,6 +29,9 @@ reference (oracle/_ref) run on the box's CPU on the same bytes, by every rank fo
   --impl reference : the reference's own CPU encoder (oracle/_ref; falls back to the oracle port) timed on
                      the host cores on the same configs; rank 0 only.
   --configs c2,c4  : subset (the headline c2 always runs).
+  --steps / --warmup : timed and untimed steps of every config.
+  --dump-outputs DIR : the compressed bytes of every config's last timed step as .npy files (dump_output), to compare
+                     two builds output for output; the inputs are seeded and the same in every run.
 """
 import argparse
 import ctypes as C
@@ -212,16 +215,23 @@ def run_reference(args, rank):
             d0 = make_stream_input("c2", 0, 1)
             per = {}
             for q in (2, 3, 4):
-                t0 = time.time(); lib.compress(d0, q, 22); dt = time.time() - t0
-                per["q%d" % q] = {"value": round(len(d0) / dt / 1e6, 2), "unit": "MB/s", "ms_per_step": round(1e3 * dt, 2), "steps": 1,
+                for _ in range(args.warmup):
+                    lib.compress(d0, q, 22)
+                t0 = time.time()
+                for _ in range(args.steps):
+                    lib.compress(d0, q, 22)
+                dt = (time.time() - t0) / args.steps
+                per["q%d" % q] = {"value": round(len(d0) / dt / 1e6, 2), "unit": "MB/s", "ms_per_step": round(1e3 * dt, 2),
+                                  "steps": args.steps, "warmup": args.warmup,
                                   "e2e": {"value": round(len(d0) / dt / 1e6, 2), "unit": "MB/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
                                   "cpu_baseline": {"value": round(len(d0) / dt / 1e6, 2), "unit": "MB/s", "cores": 1, "kind": kind,
-                                                   "sample": "the whole %d-byte stream once, 1 thread" % len(d0)}}
+                                                   "sample": "the whole %d-byte stream per step, 1 thread" % len(d0)}}
             line["sub_results"][cfg] = {"workload": WORKLOADS[cfg], "lgwin": 22, "per_quality": per}
             continue
-        v, ms, cores, sample = reference_config(cfg, lib, args.gpus, 1, 0)
+        v, ms, cores, sample = reference_config(cfg, lib, args.gpus, args.steps, args.warmup)
         line["sub_results"][cfg] = {"workload": WORKLOADS[cfg], "quality": QL[cfg][0], "lgwin": QL[cfg][1],
-                                    "value": round(v, 2), "unit": "MB/s", "ms_per_step": round(ms, 2), "steps": 1,
+                                    "value": round(v, 2), "unit": "MB/s", "ms_per_step": round(ms, 2),
+                                    "steps": args.steps, "warmup": args.warmup,
                                     "cpu_baseline": {"value": round(v, 2), "unit": "MB/s", "cores": cores, "kind": kind, "sample": sample},
                                     "e2e": {"value": round(v, 2), "unit": "MB/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
     _emit(line)
@@ -252,6 +262,32 @@ def _emit(line):
         sys.stdout.write(data.decode()); sys.stdout.flush()
     else:
         os.write(_REAL_STDOUT, data)
+
+
+DUMP_BUDGET = 60_000_000   # bytes of sampled float32 data in all; the size arrays stay below the rest of 64 MB
+
+
+def dump_sample(configs, world):
+    """Bytes kept per dumped output: DUMP_BUDGET shared by the outputs of every rank (c2, one per further config, five
+    for q234, which runs at N = 1 only)."""
+    outputs = 1 + sum(c in configs for c in ("c4", "c3", "c5", "c5q5")) + (5 if "q234" in configs and world == 1 else 0)
+    return DUMP_BUDGET // (4 * outputs * world)
+
+
+def dump_output(out_dir, name, blobs, sample):
+    """What one timed call returned in its last step: DIR/<name>_sizes.npy, the length of every compressed stream, and
+    DIR/<name>.npy, the streams' bytes laid end to end, as float32 -- all of them up to `sample` bytes, else the bytes
+    at `sample` positions drawn with a fixed seed (numpy default_rng(0), sorted), so that two builds compare
+    position by position for as long as their outputs have the same length."""
+    import numpy as np
+    if not out_dir:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    data = np.frombuffer(b"".join(blobs), np.uint8)
+    if data.size > sample:
+        data = data[np.sort(np.random.default_rng(0).choice(data.size, sample, replace=False))]
+    np.save(os.path.join(out_dir, name + ".npy"), data.astype(np.float32))
+    np.save(os.path.join(out_dir, name + "_sizes.npy"), np.array([len(b) for b in blobs], np.float64))
 
 
 # ------------------------------------------------------------------------------------------ GPU arm
@@ -324,8 +360,7 @@ def bench_stream(ctx, cfg, steps, warmup, extra_warm=True):
         h_pout = torch.zeros(cap, dtype=torch.uint8)
         if extra_warm:
             step_e2e_c_abi(h_page, h_pout)
-        dt_page, _ = ctx.timed(lambda: step_e2e_c_abi(h_page, h_pout), max(1, steps // 2))
-        dt_page *= steps / max(1, steps // 2)
+        dt_page, _ = ctx.timed(lambda: step_e2e_c_abi(h_page, h_pout), steps)
         got = bytes(h_out[:out_size].numpy().tobytes())
         d2h = out_size
     else:
@@ -338,6 +373,7 @@ def bench_stream(ctx, cfg, steps, warmup, extra_warm=True):
         got = bytes(h_mine.numpy().tobytes())
         d2h = sum(res["sizes"]) if rank == 0 else 0
     assert outs2[-1] == out_size
+    dump_output(ctx.dump, cfg if world == 1 else "%s_rank%d" % (cfg, rank), [got], ctx.dump_sample)
 
     # ---- parity of this very run against the reference, outside the timed region: every rank checks its own shard;
     # rank 0 also checks that the gathered copies are the bytes the ranks produced
@@ -471,6 +507,8 @@ def bench_c5(ctx, steps, warmup):
     ok = all(a == b for a, b in zip(got, want))
     h_dense = torch.empty(dense, dtype=torch.uint8); h_dense.copy_(d_out[:dense])
     hd = h_dense.numpy()
+    dump_output(ctx.dump, "c5" if world == 1 else "c5_rank%d" % rank,
+                [hd[int(out_off[k]):int(out_off[k]) + int(out_sz[k])].tobytes() for k in range(cnt)], ctx.dump_sample)
     ok = ok and all(bytes(hd[int(out_off[k]):int(out_off[k]) + int(out_sz[k])].tobytes()) == want[k] for k in range(cnt))
     if world > 1:
         flag = torch.tensor([1 if ok else 0], device="cuda")
@@ -534,6 +572,8 @@ def bench_c5q5(ctx, steps, warmup):
     dt, _ = ctx.timed(step, steps)
     st = brotli_b200.last_stats()
     out_total = sum(out_sizes[k] for k in range(cnt))
+    dump_output(ctx.dump, "c5q5" if world == 1 else "c5q5_rank%d" % rank, [outs[k].raw[:out_sizes[k]] for k in range(cnt)],
+                ctx.dump_sample)
     kind, lib = ref_lib()
     ncpu = max(1, (os.cpu_count() or 1) // world)
     want = [None] * cnt
@@ -568,7 +608,7 @@ def bench_c5q5(ctx, steps, warmup):
     return r
 
 
-def q234_child():
+def q234_child(steps, warmup, dump, sample):
     """Child process of the q234 sub-result: C2's input at quality 2, 3, 4 on cuda:0; prints one JSON object."""
     import torch
     import brotli_b200
@@ -595,8 +635,8 @@ def q234_child():
             sz = C.c_size_t(cap)
             assert L.BrotliEncoderCompress(q, 22, 0, n, h_in.data_ptr(), C.byref(sz), h_out.data_ptr()), "BrotliEncoderCompress failed"
             return sz.value
-        steps = 3
-        dev(); dev(); dev()                       # W = 3 warm-up steps
+        for _ in range(warmup):
+            dev()
         torch.cuda.synchronize(); t0 = time.perf_counter()
         for _ in range(steps):
             out_size = dev()
@@ -608,8 +648,9 @@ def q234_child():
             assert e2e() == out_size
         torch.cuda.synchronize(); dt2 = time.perf_counter() - t0
         got = bytes(h_out[:out_size].numpy().tobytes())
+        dump_output(dump, "q234_q%d" % q, [got], sample)
         t1 = time.time(); want = lib.compress(data, q, 22); t_cpu = time.time() - t1
-        r = {"quality": q, "lgwin": 22, "steps": steps, "warmup": 3, "input_bytes": n, "compressed_bytes": out_size,
+        r = {"quality": q, "lgwin": 22, "steps": steps, "warmup": warmup, "input_bytes": n, "compressed_bytes": out_size,
              "bit_exact": got == want, "value": round(n * steps / dt / 1e6, 2), "unit": "MB/s", "ms_per_step": round(1e3 * dt / steps, 2),
              "e2e": {"value": round(n * steps / dt2 / 1e6, 2), "unit": "MB/s", "h2d_bytes_per_step": n, "d2h_bytes_per_step": out_size,
                      "path": "BrotliEncoderCompress(host in, host out), pinned buffers"},
@@ -651,12 +692,14 @@ def q234_child():
                 C.memmove(out_sizes, caps_arr, C.sizeof(caps_arr))
                 good = L.BrotliB200CompressBatch(q, 22, cnt, in_ptrs, sizes, out_ptrs, out_sizes, 16)
                 assert good == cnt, "BrotliB200CompressBatch: %d of %d" % (good, cnt)
-            step(); step(); step()
+            for _ in range(warmup):
+                step()
             torch.cuda.synchronize(); t0 = time.perf_counter()
-            for _ in range(3):
+            for _ in range(steps):
                 step()
             torch.cuda.synchronize(); dt = time.perf_counter() - t0
             st = brotli_b200.last_stats()
+            dump_output(dump, "q234_batch_q%d" % q, [outs[k].raw[:out_sizes[k]] for k in range(cnt)], sample)
             want = [None] * cnt
             t1 = time.time()
             def work(k):
@@ -664,10 +707,10 @@ def q234_child():
                     want[i] = lib.compress(streams[i], q, 22)
             run_threads(ncpu, work)
             t_cpu = time.time() - t1
-            v = round(cnt * C5_SIZE * 3 / dt / 1e6, 2)
-            batch["q%d" % q] = {"streams": cnt, "stream_bytes": C5_SIZE, "quality": q, "lgwin": 22, "steps": 3, "warmup": 3,
+            v = round(cnt * C5_SIZE * steps / dt / 1e6, 2)
+            batch["q%d" % q] = {"streams": cnt, "stream_bytes": C5_SIZE, "quality": q, "lgwin": 22, "steps": steps, "warmup": warmup,
                                 "bit_exact": all(outs[k].raw[:out_sizes[k]] == want[k] for k in range(cnt)),
-                                "value": v, "unit": "MB/s", "ms_per_step": round(1e3 * dt / 3, 2),
+                                "value": v, "unit": "MB/s", "ms_per_step": round(1e3 * dt / steps, 2),
                                 "e2e": {"value": v, "unit": "MB/s", "h2d_bytes_per_step": cnt * C5_SIZE,
                                         "d2h_bytes_per_step": sum(out_sizes[k] for k in range(cnt)),
                                         "path": "BrotliB200CompressBatch(host pointer arrays): value == e2e for this call"},
@@ -682,10 +725,13 @@ def q234_child():
     sys.stdout.flush()
 
 
-def bench_q234():
-    """Runs q234_child in a process of its own (time limit 5 minutes; it needs about two): a crash or a hang of the newest
-    path ends the child, not the bench."""
-    p = subprocess.run([sys.executable, os.path.abspath(__file__), "--q234-child"], stdout=subprocess.PIPE, timeout=300)
+def bench_q234(steps, warmup, dump, sample):
+    """Runs q234_child in a process of its own (time limit 5 minutes and 20 s per step; it needs about two minutes at 3
+    steps): a crash or a hang of the newest path ends the child, not the bench."""
+    cmd = [sys.executable, os.path.abspath(__file__), "--q234-child", "--steps", str(steps), "--warmup", str(warmup)]
+    if dump:
+        cmd += ["--dump-outputs", dump, "--dump-sample", str(sample)]
+    p = subprocess.run(cmd, stdout=subprocess.PIPE, timeout=300 + 20 * (steps + warmup))
     lines = [l for l in p.stdout.decode("utf-8", "replace").splitlines() if l.startswith("{")]
     if p.returncode != 0 or not lines:
         raise RuntimeError("q234 child exited with %d" % p.returncode)
@@ -693,17 +739,21 @@ def bench_q234():
 
 
 def main():
-    if "--q234-child" in sys.argv:
-        q234_child()
-        return
-    _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every config")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed steps in front of them")
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--configs", default="c2,c4,c3,c5,c5q5,q234")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the compressed bytes of every config's last timed step "
+                    "under DIR (dump_output)")
+    ap.add_argument("--q234-child", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-sample", type=int, default=0, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.q234_child:
+        q234_child(args.steps, args.warmup, args.dump_outputs, args.dump_sample)
+        return
+    _claim_stdout()
     args.configs = [c for c in args.configs.split(",") if c in WORKLOADS]
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -721,7 +771,8 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     ctx = Ctx()
-    ctx.L, ctx.rank, ctx.world = brotli_b200.lib(), rank, world
+    ctx.L, ctx.rank, ctx.world, ctx.dump = brotli_b200.lib(), rank, world, args.dump_outputs
+    ctx.dump_sample = dump_sample(args.configs, world)
 
     def barrier():
         torch.cuda.synchronize()
@@ -758,16 +809,14 @@ def main():
     for cfg in args.configs:
         t0 = time.time()
         try:
-            if cfg == "c4":
-                sub[cfg] = bench_stream(ctx, "c4", 1, 1, extra_warm=False)
-            elif cfg == "c3":
-                sub[cfg] = bench_stream(ctx, "c3", 3, 1, extra_warm=False)
+            if cfg in ("c4", "c3"):
+                sub[cfg] = bench_stream(ctx, cfg, args.steps, args.warmup, extra_warm=False)
             elif cfg == "c5":
-                sub[cfg] = bench_c5(ctx, 5, 2)
+                sub[cfg] = bench_c5(ctx, args.steps, args.warmup)
             elif cfg == "c5q5":
-                sub[cfg] = bench_c5q5(ctx, 5, 2)
+                sub[cfg] = bench_c5q5(ctx, args.steps, args.warmup)
             elif cfg == "q234" and world == 1:
-                sub[cfg] = bench_q234()
+                sub[cfg] = bench_q234(args.steps, args.warmup, args.dump_outputs, ctx.dump_sample)
         except Exception as e:      # a sub-result must not take the headline line with it (one rank: the others would hang)
             if world > 1:
                 raise

@@ -1,14 +1,22 @@
 """ctypes loaders for the checker libraries (oracle/ and oracle/_ref) and the product
-C-ABI (brotli_b200/libbrotlienc_b200.so).  Test infrastructure only."""
+C-ABI (brotli_b200/libbrotlienc_b200.so), and RecordedRef, the reference's recorded
+outputs the suite compares against.  Test infrastructure only."""
+import atexit
 import ctypes as C
+import hashlib
+import json
 import os
+import subprocess
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_SO = os.path.join(ROOT, "oracle", "_ref", "libbrotli_ref.so")
+REF_CLI = os.path.join(ROOT, "oracle", "_ref", "brotli_cli_ref")
+B200_CLI = os.path.join(ROOT, "oracle", "_ref", "brotli_cli_b200")    # the same CLI linked against this library
 PROBE_SO = os.path.join(ROOT, "oracle", "_ref", "libbrotli_probe.so")
 ORACLE_SO = os.path.join(ROOT, "oracle", "liboracle.so")
 TABLES = os.path.join(ROOT, "brotli_b200", "data", "brotli_tables.bin")
 PRODUCT_SO = os.path.join(ROOT, "brotli_b200", "libbrotlienc_b200.so")
+REFERENCE_OUTPUTS = os.path.join(ROOT, "tests", "golden", "reference_outputs.json")
 
 _u8p = C.POINTER(C.c_uint8)
 
@@ -32,7 +40,7 @@ def zeroed_malloc():
 
 
 class Ref:
-    """The unmodified reference compiled from /root/reference (oracle/Makefile)."""
+    """The unmodified reference, compiled from its sources into oracle/_ref by oracle/Makefile."""
 
     def __init__(self, path=REF_SO):
         self.lib = C.CDLL(path, mode=os.RTLD_LOCAL)
@@ -103,11 +111,11 @@ class Oracle:
         return out.raw[:out_n.value]
 
 
-def ref_compress_stream(ref, data, quality, lgwin, chunk, out_buf=1 << 19):
-    """Drives the reference's streaming API the way c/tools/brotli.c:1357 does: PROCESS calls of
-    `chunk` bytes, FINISH once the input is exhausted (an extra empty call when the size is a
-    multiple of `chunk`, like feof() after a full read)."""
-    L = ref.lib
+def cli_compress_stream(L, data, quality, lgwin, chunk, out_buf=1 << 19, size_hint=0):
+    """Drives the streaming API of library L (the reference's or this project's) the way c/tools/brotli.c:1357 does:
+    PROCESS calls of `chunk` bytes, FINISH once the input is exhausted (an extra empty call when the size is a multiple
+    of `chunk`, like feof() after a full read), a caller output buffer of `out_buf` bytes drained whenever it is full,
+    until BrotliEncoderIsFinished; `size_hint` as the CLI sets it for an input file (c/tools/brotli.c:1448)."""
     L.BrotliEncoderCreateInstance.restype = C.c_void_p
     L.BrotliEncoderCreateInstance.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.BrotliEncoderSetParameter.argtypes = [C.c_void_p, C.c_int, C.c_uint32]
@@ -118,6 +126,8 @@ def ref_compress_stream(ref, data, quality, lgwin, chunk, out_buf=1 << 19):
     s = L.BrotliEncoderCreateInstance(None, None, None)
     L.BrotliEncoderSetParameter(s, 1, quality)
     L.BrotliEncoderSetParameter(s, 2, lgwin)
+    if size_hint:
+        L.BrotliEncoderSetParameter(s, 5, min(size_hint, 1 << 30))
     src = C.create_string_buffer(data, max(1, len(data)))
     dst = C.create_string_buffer(out_buf)
     out = bytearray()
@@ -175,3 +185,110 @@ def ref_stream_ops(ref, data, quality, lgwin, sizes, ops, out_buf=1 << 16, param
                 break
     L.BrotliEncoderDestroyInstance(s)
     return bytes(out)
+
+
+def _digest(b):
+    """Length and the first 128 bits of the SHA-256 of a byte string (or of a RefOutput standing for one)."""
+    if isinstance(b, RefOutput):
+        return b.digest
+    return "%d:%s" % (len(b), hashlib.sha256(bytes(b)).hexdigest()[:32])
+
+
+class RefOutput(object):
+    """A byte string the reference produced, known by its digest: compares equal to bytes with that digest."""
+
+    def __init__(self, digest):
+        self.digest = digest
+
+    def __len__(self):
+        return int(self.digest.split(":")[0])
+
+    def __eq__(self, other):
+        if isinstance(other, (bytes, bytearray, RefOutput)):
+            return _digest(other) == self.digest
+        return NotImplemented
+
+    def __repr__(self):
+        return "RefOutput(%s)" % self.digest
+
+
+_RECORD_PATH = os.environ.get("BROTLI_RECORD_REFERENCE")
+_recorded = {}
+_table = None
+
+
+def _write_recorded():
+    table = json.load(open(_RECORD_PATH)) if os.path.exists(_RECORD_PATH) else {}
+    table.update(_recorded)
+    with open(_RECORD_PATH, "w") as f:
+        json.dump(table, f, indent=0, sort_keys=True)
+        f.write("\n")
+
+
+class RecordedRef(object):
+    """The reference encoder / decoder / CLI as the suite calls them, answered from tests/golden/reference_outputs.json:
+    for every call the tests make, the digest of what the unmodified reference returned (RefOutput; integers as they
+    are), keyed by the call and the digests of its inputs.  The suite so compares against the reference without its
+    sources or a build of them; a call that was not recorded (new arguments, or an input that drifted) fails.
+
+    To record: build oracle/_ref (BROTLI_REFERENCE=<google/brotli checkout> python __graft_entry__.py) and run the tests
+    that use this class with BROTLI_RECORD_REFERENCE=<json file>: the calls then go to the reference, the tests compare
+    against its real output, and the digests are merged into that file when the process exits."""
+
+    def __init__(self):
+        global _table
+        if _RECORD_PATH:
+            self.live = Ref()
+            if _table is None:
+                _table = {}
+                atexit.register(_write_recorded)
+        else:
+            self.live = None
+            if _table is None:
+                _table = json.load(open(REFERENCE_OUTPUTS))
+
+    def _answer(self, call, inputs, run):
+        key = hashlib.sha256(json.dumps([call, [_digest(x) for x in inputs]]).encode()).hexdigest()[:20]
+        if self.live is not None:
+            out = run(self.live)
+            _recorded[key] = out if isinstance(out, int) else _digest(out)
+            return out
+        assert key in _table, "no recorded reference output for %r on inputs %r" % (call, [_digest(x) for x in inputs])
+        v = _table[key]
+        return v if isinstance(v, int) else RefOutput(v)
+
+    def compress(self, data, quality, lgwin, mode=0):
+        return self._answer(["compress", quality, lgwin, mode], [data], lambda r: r.compress(data, quality, lgwin, mode))
+
+    def decompress(self, comp, max_out):
+        return self._answer(["decompress", max_out], [comp], lambda r: r.decompress(comp, max_out))
+
+    def max_compressed_size(self, n):
+        return self._answer(["max_compressed_size", n], [], lambda r: int(r.lib.BrotliEncoderMaxCompressedSize(n)))
+
+    def stream_ops(self, data, quality, lgwin, sizes, ops, params=None):
+        """ref_stream_ops: CompressStream with an explicit list of (size, op) calls."""
+        call = ["stream_ops", quality, lgwin, list(sizes), list(ops), sorted((params or {}).items())]
+        return self._answer(call, [data], lambda r: ref_stream_ops(r, data, quality, lgwin, sizes, ops, params=params))
+
+    def compress_stream(self, data, quality, lgwin, chunk):
+        """cli_compress_stream: PROCESS calls of `chunk` bytes, then FINISH."""
+        return self._answer(["compress_stream", quality, lgwin, chunk], [data],
+                            lambda r: cli_compress_stream(r.lib, data, quality, lgwin, chunk))
+
+    def cli(self, args, data, from_file):
+        """The reference's CLI (oracle/_ref/brotli_cli_ref) run with `args` on `data` (run_cli)."""
+        return self._answer(["cli", args, from_file], [data], lambda r: run_cli(REF_CLI, args, data, from_file))
+
+
+def run_cli(path, args, data, from_file):
+    """The CLI of c/tools/brotli.c at `path` run with `args` on `data`, read from a file (the CLI sets the size hint
+    and may shrink the window from the file's length) or from a pipe; returns what it wrote."""
+    if not from_file:
+        return subprocess.run([path] + args + ["-c"], input=data, stdout=subprocess.PIPE, check=True).stdout
+    import tempfile
+    with tempfile.TemporaryDirectory() as tmp:
+        src, dst = os.path.join(tmp, "in"), os.path.join(tmp, "in.br")
+        open(src, "wb").write(data)
+        subprocess.check_call([path] + args + ["-f", "-o", dst, src])
+        return open(dst, "rb").read()

@@ -1,5 +1,5 @@
 """GPU suite (-m gpu): the CUDA path, called through the C ABI, against the golden vectors of the
-compiled reference, the oracle, and -- where it travelled -- oracle/_ref itself.  Bit-exact."""
+compiled reference, the oracle, and the reference's recorded outputs (brotli_libs.RecordedRef).  Bit-exact."""
 import ctypes as C
 import hashlib
 import json
@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-from brotli_libs import REF_SO, Oracle, Ref, ref_compress_stream, ref_stream_ops
+from brotli_libs import Oracle, RecordedRef
 from golden_cases import make_case
 
 pytestmark = pytest.mark.gpu
@@ -96,13 +96,12 @@ def _drive(b200, d, q, w, sizes, ops):
     return out
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_streaming_flush_and_metadata(b200):
     """FLUSH and EMIT_METADATA at quality 5..9 (encode.c:1356, :1549): byte-identical to the reference's CompressStream for
     the same call sequence -- flushes inside and at block boundaries, a flush / metadata before any input, metadata between
     data, repeated operations at one position, FINISH without input behind a full block, and everything flushed bytewise."""
     from corpus import synth_binary, synth_text
-    ref = Ref()
+    ref = RecordedRef()
     for d in (synth_text(700000, 61), synth_binary(900000, 62)):
         n = len(d)
         for q, w in ((5, 22), (9, 24), (6, 18)):
@@ -119,7 +118,7 @@ def test_streaming_flush_and_metadata(b200):
                 if sum(a for a, op in zip(sizes, ops) if op != 3) > n:
                     continue
                 # metadata payloads are taken from the same buffer; they are not stream input
-                want = ref_stream_ops(ref, d, q, w, sizes, ops)
+                want = ref.stream_ops(d, q, w, sizes, ops)
                 got = _drive(b200, d, q, w, sizes, ops)
                 assert got == want, (q, w, sizes, ops, len(got), len(want))
                 # the flushed prefixes really decode: cut the stream behind its last flush and finish it by hand
@@ -132,12 +131,11 @@ def test_streaming_flush_and_metadata(b200):
     assert ref.decompress(part + rest, len(d)) == d
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_lgblock_and_context_modeling_parameters(b200):
     """BROTLI_PARAM_LGBLOCK (encode.h:184, quality.h:76) and BROTLI_PARAM_DISABLE_LITERAL_CONTEXT_MODELING (encode.h:191,
     encode.c:561) through the streaming API, against the reference with the same parameters."""
     from corpus import synth_web
-    ref = Ref()
+    ref = RecordedRef()
     L = b200.lib()
     d = synth_web(1500000, 65)
     for q, w in ((5, 22), (9, 24)):
@@ -147,7 +145,7 @@ def test_lgblock_and_context_modeling_parameters(b200):
                 prm[3] = lgb
             if dis:
                 prm[4] = 1
-            want = ref_stream_ops(ref, d, q, w, [700000, len(d) - 700000], [1, 2], params=prm)
+            want = ref.stream_ops(d, q, w, [700000, len(d) - 700000], [1, 2], params=prm)
             c = b200.Compressor(quality=q, lgwin=w, lgblock=lgb)
             if dis:
                 assert L.BrotliEncoderSetParameter(c._s, 4, 1)
@@ -155,13 +153,12 @@ def test_lgblock_and_context_modeling_parameters(b200):
             assert got == want, (q, w, lgb, dis)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_stream_offset_stitches_shards(b200):
     """SURVEY.md 8e: one valid stream out of independently compressed shards -- every shard but the first is compressed with
     BROTLI_PARAM_STREAM_OFFSET = its start (encode.h:231), every shard but the last ends with FLUSH instead of FINISH.
     Each shard equals the reference run with the same parameters and calls; the concatenation decodes to the input."""
     from corpus import synth_web
-    ref = Ref()
+    ref = RecordedRef()
     L = b200.lib()
     d = synth_web(1800000, 68)
     cuts = [0, 500000, 1300001, len(d)]
@@ -171,7 +168,7 @@ def test_stream_offset_stitches_shards(b200):
             part = d[cuts[i]:cuts[i + 1]]
             last = i == 2
             prm = {9: cuts[i]} if i else {}
-            want = ref_stream_ops(ref, part, q, w, [len(part)], [2 if last else 1], params=prm)
+            want = ref.stream_ops(part, q, w, [len(part)], [2 if last else 1], params=prm)
             c = b200.Compressor(quality=q, lgwin=w)
             if i:
                 # (the Compressor has not been used yet: parameters can still be set)
@@ -283,27 +280,25 @@ def test_batch_of_small_streams(b200):
         assert got[k] == ora.compress(x, 5, 22), k
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_full_size_properties(b200):
-    """BASELINE.json's full size (100 MB, q5, lgwin 22): equality with the reference run on the
-    box's CPU, and the size-independent property decode(encode(x)) == x via the reference decoder."""
+    """BASELINE.json's full size (100 MB, q5, lgwin 22): equality with the reference's output,
+    and the size-independent property decode(encode(x)) == x via the reference decoder (both recorded)."""
     from corpus import synth_text
-    ref = Ref()
+    ref = RecordedRef()
     d = synth_text(100_000_000)
     out = b200.compress_oneshot(d, 5, 22)
     assert ref.decompress(out, len(d)) == d
     assert out == ref.compress(d, 5, 22)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_q9_ring_wrap_and_nonsettling_inputs(b200):
     """Quality 9 / lgwin 24 beyond the 32 MiB ring buffer of the reference (BASELINE config C4's path: H6, 256-entry
     rings, 256 KiB input blocks), on the Silesia-shaped binary mix, and inputs whose parse never settles by itself --
     uniform noise (the sparse search's position phase runs through the whole input) and int32 random walks.  The
-    encoder must never fail (encode.c:1340-1353) and must equal the reference run on the box."""
+    encoder must never fail (encode.c:1340-1353) and must equal the reference's output (recorded)."""
     import numpy as np
     from corpus import synth_binary
-    ref = Ref()
+    ref = RecordedRef()
     cases = [("binary mix 48 MiB", synth_binary(48 << 20, 91), 9, 24),
              ("uniform noise 24 MiB", np.random.RandomState(92).randint(0, 256, 24 << 20, dtype=np.uint8).tobytes(), 9, 24),
              ("uniform noise 16 MiB q5", np.random.RandomState(93).randint(0, 256, 16 << 20, dtype=np.uint8).tobytes(), 5, 22),
@@ -313,12 +308,11 @@ def test_q9_ring_wrap_and_nonsettling_inputs(b200):
         assert out == ref.compress(d, q, w), name
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_config3_slice_and_config5_streams(b200):
     """BASELINE config C3 (web mix, quality 5, lgwin 22) on a 256 MiB slice, and config C5 on 1000 of its 64 KiB streams
-    (quality 1, one device batch), each against the reference run on the box."""
+    (quality 1, one device batch), each against the reference's recorded outputs."""
     from corpus import synth_web
-    ref = Ref()
+    ref = RecordedRef()
     web = synth_web(256 << 20)
     out = b200.compress_oneshot(web, 5, 22)
     assert out == ref.compress(web, 5, 22)
@@ -328,50 +322,43 @@ def test_config3_slice_and_config5_streams(b200):
         assert got[i] == ref.compress(s, 1, 22), i
 
 
-def test_cli_dropin(b200, tmp_path):
-    """The reference's own CLI (c/tools/brotli.c, unmodified) linked against this library instead of
-    libbrotlienc produces the same file as the CLI linked against the reference encoder."""
-    import subprocess
-    from brotli_libs import ROOT
-    cli_ref = os.path.join(ROOT, "oracle", "_ref", "brotli_cli_ref")
-    cli_b200 = os.path.join(ROOT, "oracle", "_ref", "brotli_cli_b200")
-    if not (os.path.exists(cli_ref) and os.path.exists(cli_b200)):
-        pytest.skip("CLI binaries were not built (oracle/Makefile ref)")
+def _check_cli(b200, data, q, w, from_file):
+    """The reference's CLI (c/tools/brotli.c, unmodified) on `data` with `-q q -w w`: what it writes when linked against this
+    library must equal what it writes when linked against the reference encoder (recorded).  The CLI linked against this
+    library (oracle/_ref/brotli_cli_b200) runs where build() could compile it from the reference; the CLI's own call
+    loop (brotli_libs.cli_compress_stream: 512 KiB reads, a 512 KiB output buffer drained when full, the size hint of an
+    input file) runs over this library everywhere."""
+    from brotli_libs import B200_CLI, cli_compress_stream, run_cli
+    args = ["-q", str(q), "-w", str(w)]
+    want = RecordedRef().cli(args, data, from_file)
+    assert len(want) > 0
+    got = cli_compress_stream(b200.lib(), data, q, w, 1 << 19, size_hint=len(data) if from_file else 0)
+    assert got == want, ("CLI call loop", len(data), q, w, from_file)
+    if os.path.exists(B200_CLI):
+        assert run_cli(B200_CLI, args, data, from_file) == want, ("brotli_cli_b200", len(data), q, w, from_file)
+
+
+def test_cli_dropin(b200):
+    """The reference's own CLI (c/tools/brotli.c, unmodified) linked against this library instead of libbrotlienc
+    produces the same file as the CLI linked against the reference encoder (_check_cli)."""
     from corpus import synth_text
-    src = tmp_path / "in.txt"
-    src.write_bytes(synth_text(3_000_000, 77))
-    outs = []
-    for cli in (cli_ref, cli_b200):
-        dst = tmp_path / (os.path.basename(cli) + ".br")
-        subprocess.check_call([cli, "-q", "5", "-w", "22", "-f", "-o", str(dst), str(src)])
-        outs.append(dst.read_bytes())
-    assert outs[0] == outs[1] and len(outs[0]) > 0
+    _check_cli(b200, synth_text(3_000_000, 77), 5, 22, True)
 
 
-def test_cli_dropin_stdin(b200, tmp_path):
+def test_cli_dropin_stdin(b200):
     """The same CLI reading a PIPE: no size hint (c/tools/brotli.c:1448-1452), 512 KiB PROCESS calls, an input that is an
     exact multiple of the read size (FINISH arrives without input behind a full block), quality 5 and 9."""
-    import subprocess
-    from brotli_libs import ROOT
-    cli_ref = os.path.join(ROOT, "oracle", "_ref", "brotli_cli_ref")
-    cli_b200 = os.path.join(ROOT, "oracle", "_ref", "brotli_cli_b200")
-    if not (os.path.exists(cli_ref) and os.path.exists(cli_b200)):
-        pytest.skip("CLI binaries were not built (oracle/Makefile ref)")
     from corpus import synth_web
     for n, q, w in ((3 * 524288, 5, 22), (2_500_001, 9, 24), (700_000, 6, 18)):
-        data = synth_web(n, 78)
-        outs = [subprocess.run([cli, "-q", str(q), "-w", str(w), "-c"], input=data, stdout=subprocess.PIPE, check=True).stdout
-                for cli in (cli_ref, cli_b200)]
-        assert outs[0] == outs[1] and len(outs[0]) > 0, (n, q, w)
+        _check_cli(b200, synth_web(n, 78), q, w, False)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_one_shot_wrapper_rules(b200):
     """encode.c:1296-1353 / quality.h:60: quality 1 with lgwin above 24 is sanitised to 24 (no large window at quality <= 2);
     an output buffer that is too small fails; an incompressible input still fits BrotliEncoderMaxCompressedSize."""
     import numpy as np
     from corpus import synth_text
-    ref = Ref()
+    ref = RecordedRef()
     L = b200.lib()
     d = synth_text(200000, 66)
     assert b200.compress_oneshot(d, 1, 27) == ref.compress(d, 1, 27) == ref.compress(d, 1, 24)
@@ -431,34 +418,20 @@ def test_q1_streaming_call_pattern(b200):
         out += c.finish()
         calls = [a for a in sizes if a] + [0]
         assert out == ora.compress_q1_stream(d, 22, calls), sizes
-    if os.path.exists(REF_SO):
-        ref = Ref()
-        c = b200.Compressor(quality=1, lgwin=18)
-        out = b""
-        for o in range(0, len(d), 1 << 19):
-            out += c.process(d[o:o + (1 << 19)])
-        out += c.finish()
-        assert out == ref_compress_stream(ref, d, 1, 18, 1 << 19)
-        assert ref.decompress(out, len(d)) == d
+    ref = RecordedRef()
+    c = b200.Compressor(quality=1, lgwin=18)
+    out = b""
+    for o in range(0, len(d), 1 << 19):
+        out += c.process(d[o:o + (1 << 19)])
+    out += c.finish()
+    assert out == ref.compress_stream(d, 1, 18, 1 << 19)
+    assert ref.decompress(out, len(d)) == d
 
 
-def test_q1_cli_dropin(b200, tmp_path):
-    import subprocess
-    from brotli_libs import ROOT
-    cli_ref = os.path.join(ROOT, "oracle", "_ref", "brotli_cli_ref")
-    cli_b200 = os.path.join(ROOT, "oracle", "_ref", "brotli_cli_b200")
-    if not (os.path.exists(cli_ref) and os.path.exists(cli_b200)):
-        pytest.skip("CLI binaries were not built (oracle/Makefile ref)")
+def test_q1_cli_dropin(b200):
     from corpus import synth_web
     for n in (3_000_000, 1 << 20):       # the second one ends exactly on a 512 KiB read: empty FINISH call
-        src = tmp_path / ("in%d.html" % n)
-        src.write_bytes(synth_web(n, 78))
-        outs = []
-        for cli in (cli_ref, cli_b200):
-            dst = tmp_path / (os.path.basename(cli) + ".br")
-            subprocess.check_call([cli, "-q", "1", "-w", "22", "-f", "-o", str(dst), str(src)])
-            outs.append(dst.read_bytes())
-        assert outs[0] == outs[1] and len(outs[0]) > 0
+        _check_cli(b200, synth_web(n, 78), 1, 22, True)
 
 
 def test_q1_flush(b200):
@@ -482,11 +455,9 @@ def test_q1_flush(b200):
                 else:
                     out += c._stream(piece, c._FINISH)
             assert out == ora.compress_q1_stream(d, w, sizes, ops), (sizes, ops, w)
-            if os.path.exists(REF_SO):
-                assert out == ref_stream_ops(Ref(), d, 1, w, sizes, ops)
+            assert out == RecordedRef().stream_ops(d, 1, w, sizes, ops)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_q1_stream_beyond_one_device_segment(b200):
     """Quality 1 has no stream-size limit: input above one device segment (128 MiB) runs as several, a segment that
     neither flushes nor finishes ends mid-byte and the next starts behind its pending bits (br_api.cc q1_run).
@@ -499,7 +470,7 @@ def test_q1_stream_beyond_one_device_segment(b200):
     d[idx] = rng.integers(0, 256, idx.size, dtype=np.uint8)
     d[(1 << 27) - 3_000_000:(1 << 27) + 3_000_000] = rng.integers(0, 256, 6_000_000, dtype=np.uint8)   # raw fragments across a cut
     d = d.tobytes()
-    ref = Ref()
+    ref = RecordedRef()
     for w in (22, 18):
         assert b200.compress_oneshot(d, 1, w) == ref.compress(d, 1, w), w
     step = (24 << 20) + 1
@@ -510,7 +481,7 @@ def test_q1_stream_beyond_one_device_segment(b200):
     for a, op in zip(sizes, ops):
         piece = d[o:o + a]; o += a
         out.append(c.process(piece) if op == 0 else c._stream(piece, c._FINISH))
-    assert b"".join(out) == ref_stream_ops(ref, d, 1, 22, sizes, ops, out_buf=1 << 24)
+    assert b"".join(out) == ref.stream_ops(d, 1, 22, sizes, ops)
 
 
 def test_fuzz_gpu(b200):

@@ -1,12 +1,12 @@
 """CPU suite, part 1: the oracle (oracle/brotli_oracle.c) against the golden vectors made from the
-compiled reference, and -- where oracle/_ref is present -- against the reference itself."""
+compiled reference, and against the reference's recorded outputs (brotli_libs.RecordedRef)."""
 import hashlib
 import json
 import os
 
 import pytest
 
-from brotli_libs import REF_SO, Oracle, Ref, ref_compress_stream
+from brotli_libs import PRODUCT_SO, Oracle, RecordedRef
 from golden_cases import make_case
 
 GOLDEN = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "golden.json")))
@@ -48,9 +48,8 @@ def test_oracle_matches_golden(oracle, g):
     assert hashlib.sha256(out).hexdigest() == g["out_sha256"]
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
 def test_oracle_matches_reference_and_roundtrips(oracle):
-    ref = Ref()
+    ref = RecordedRef()
     for g in FAST[:12]:
         d = make_case(g)
         a = ref.compress(d, g["q"], g["lgwin"])
@@ -58,12 +57,17 @@ def test_oracle_matches_reference_and_roundtrips(oracle):
         assert ref.decompress(a, len(d)) == d
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
 def test_empty_input_and_bounds():
-    ref = Ref()
+    """The reference's output for empty input, and its BrotliEncoderMaxCompressedSize, which the product's must equal."""
+    import ctypes as C
+    ref = RecordedRef()
     assert ref.compress(b"", 5, 22) == b"\x06"
+    lib = C.CDLL(PRODUCT_SO, mode=os.RTLD_LOCAL)      # built by build(); its host-only entry points need no GPU
+    lib.BrotliEncoderMaxCompressedSize.restype = C.c_size_t
+    lib.BrotliEncoderMaxCompressedSize.argtypes = [C.c_size_t]
     for n in (0, 1, 100, 1 << 14, (1 << 24) + 5):
-        assert ref.lib.BrotliEncoderMaxCompressedSize(n) >= n
+        assert ref.max_compressed_size(n) >= n
+        assert lib.BrotliEncoderMaxCompressedSize(n) == ref.max_compressed_size(n), n
 
 
 def test_fast_log2_table(oracle):
@@ -76,12 +80,11 @@ def test_fast_log2_table(oracle):
     assert oracle.lib.oracle_fast_log2(4096) == 12.0
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
 def test_q1_oracle_against_reference(oracle):
     """Quality 1 (compress_fragment_two_pass.c): one-shot calls over every table size / min_match the
     reference can pick, and the streaming call pattern of c/tools/brotli.c (512 KiB PROCESS calls)."""
     from corpus import synth_binary, synth_text, synth_web
-    ref = Ref()
+    ref = RecordedRef()
     base = synth_web(3_000_000, 51)
     for n in (0, 1, 15, 16, 17, 255, 256, 257, 1000, 5000, 40000, 65536, 131072, 131073, 300000, 1 << 20, 3_000_000):
         for w in (10, 16, 18, 22, 24):
@@ -96,15 +99,14 @@ def test_q1_oracle_against_reference(oracle):
         if n % chunk == 0:
             calls.append(0)
         for w in (16, 22):
-            assert oracle.compress_q1_stream(d, w, calls) == ref_compress_stream(ref, d, 1, w, chunk), (n, w)
+            assert oracle.compress_q1_stream(d, w, calls) == ref.compress_stream(d, 1, w, chunk), (n, w)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref not built")
 def test_q234_oracle_against_reference(oracle):
     """Qualities 2..4 (H2 / H3 / H4 / H54, fast / trivial / context-free meta-blocks): oracle groundwork for
     SURVEY.md 8f rank 1, pinned against the reference over window sizes and hasher switches."""
     from corpus import synth_binary, synth_web
-    ref = Ref()
+    ref = RecordedRef()
     base = synth_web(2_200_000, 71)
     for n in (0, 1, 7, 8, 9, 100, 5000, 16384, 16385, 70000, 300000, (1 << 20) - 1, 1 << 20, 2_200_000):
         for q in (2, 3, 4):

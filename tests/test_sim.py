@@ -196,18 +196,16 @@ def _sim_cuts(sim, d, q, w, hint, cuts, kinds, is_final, finish_empty=0, lgblock
 def test_sim_flush_cuts_and_parameters(sim):
     """The device code with the input cut by FLUSH operations (encode.c:1356, :1700), with FINISH arriving without input
     behind a full block (encode.c:520), and with BROTLI_PARAM_LGBLOCK / DISABLE_LITERAL_CONTEXT_MODELING, against the
-    reference's CompressStream driven with the same calls (needs oracle/_ref)."""
-    from brotli_libs import REF_SO, Ref, ref_stream_ops
-    if not os.path.exists(REF_SO):
-        pytest.skip("oracle/_ref not built")
+    reference's CompressStream driven with the same calls (recorded: brotli_libs.RecordedRef)."""
+    from brotli_libs import RecordedRef
     from corpus import synth_binary, synth_text, synth_web
-    ref = Ref()
+    ref = RecordedRef()
     for d in (synth_text(400000, 3), synth_binary(600000, 5)):
         n = len(d)
         for q, w in ((5, 22), (9, 24), (7, 19)):
             bs = 1 << (18 if (q >= 9 and w >= 18) else 16)
             for sizes, ops in (([100000, 50000, n - 150000], [0, 1, 2]), ([bs, 0, n - bs, 0], [0, 1, 1, 2]), ([100, n - 100, 0], [1, 0, 2])):
-                want = ref_stream_ops(ref, d, q, w, sizes, ops)
+                want = ref.stream_ops(d, q, w, sizes, ops)
                 pos, cuts, acc, fixed, hint = 0, [], 0, False, 0
                 for a, op in zip(sizes, ops):
                     if not fixed and (op != 0 or acc + a >= bs):   # encode.c:1619: the size hint freezes at the first EncodeData
@@ -225,7 +223,7 @@ def test_sim_flush_cuts_and_parameters(sim):
     d = synth_web(1_400_000, 3)
     for q, w in ((9, 24), (7, 18)):
         for sizes, ops in (([500000, 0, 900000, 0], [1, 1, 0, 2]), ([2, 700000, 699998], [1, 1, 2])):
-            want = ref_stream_ops(ref, d, q, w, sizes, ops)
+            want = ref.stream_ops(d, q, w, sizes, ops)
             cuts, pos = [], 0
             for a, op in zip(sizes, ops):
                 pos += a
@@ -234,7 +232,7 @@ def test_sim_flush_cuts_and_parameters(sim):
             assert _sim_cuts(sim, d, q, w, sizes[0], cuts, [1] * len(cuts), 1) == want, (q, w, sizes)
     d = synth_web(2 * 262144, 9)
     for q, w in ((5, 22), (9, 24)):
-        want = ref_stream_ops(ref, d, q, w, [len(d), 0], [0, 2])          # FINISH without input behind full blocks
+        want = ref.stream_ops(d, q, w, [len(d), 0], [0, 2])          # FINISH without input behind full blocks
         assert _sim_cuts(sim, d, q, w, 1 << (18 if q == 9 else 16), [], [], 1, finish_empty=1) == want
         for lgb, dis in ((0, 1), (17, 0), (20, 1), (24, 0)):
             prm = {}
@@ -242,7 +240,7 @@ def test_sim_flush_cuts_and_parameters(sim):
                 prm[3] = lgb
             if dis:
                 prm[4] = 1
-            want = ref_stream_ops(ref, d, q, w, [len(d)], [2], params=prm)
+            want = ref.stream_ops(d, q, w, [len(d)], [2], params=prm)
             assert _sim_cuts(sim, d, q, w, len(d), [], [], 1, lgblock=lgb, disable_ctx=dis) == want, (q, w, lgb, dis)
 
 
@@ -379,15 +377,13 @@ def test_sim_stream_offset(sim):
     """BROTLI_PARAM_STREAM_OFFSET (encode.h:231, the sanctioned way to stitch shards into one stream, SURVEY.md 8e): no
     window bits, poisoned distance cache (encode.c:656), dictionary distances counted from the virtual start
     (backward_references_inc.h:94), and the first two bytes flushed on their own (encode.c:1704) -- against the reference."""
-    from brotli_libs import REF_SO, Ref, ref_stream_ops
-    if not os.path.exists(REF_SO):
-        pytest.skip("oracle/_ref not built")
+    from brotli_libs import RecordedRef
     from corpus import synth_text, synth_web
-    ref = Ref()
+    ref = RecordedRef()
     for d in (synth_text(300000, 4), synth_web(500000, 10)):
         for q, w in ((5, 22), (9, 24), (6, 18)):
             for off in (1, 1000, 1 << 20, 1 << 30):
-                want = ref_stream_ops(ref, d, q, w, [len(d)], [2], params={9: off})
+                want = ref.stream_ops(d, q, w, [len(d)], [2], params={9: off})
                 got = _sim_cuts(sim, d, q, w, len(d), [2], [1], 1, stream_offset=off, with_header=0)
                 assert got == want, (q, w, off, len(got), len(want))
 
@@ -443,17 +439,15 @@ def test_sim_q234_flush_cuts(sim):
     """Qualities 2..4 with the input cut by FLUSH operations, against the reference's CompressStream driven with the same
     calls: input blocks of 1 << 14 bytes below quality 4 (quality.h:81), the MAX_NUM_DELAYED_SYMBOLS flush rule
     (encode.c:1152), FINISH without input behind a full block."""
-    from brotli_libs import REF_SO, Ref, ref_stream_ops
-    if not os.path.exists(REF_SO):
-        pytest.skip("oracle/_ref not built")
+    from brotli_libs import RecordedRef
     from corpus import synth_binary, synth_text
-    ref = Ref()
+    ref = RecordedRef()
     for d in (synth_text(300000, 3), synth_binary(400000, 5)):
         n = len(d)
         for q, w in ((2, 22), (3, 18), (4, 22), (4, 12)):
             bs = 1 << (14 if q < 4 else 16)
             for sizes, ops in (([100000, 50000, n - 150000], [0, 1, 2]), ([bs, 0, n - bs, 0], [0, 1, 1, 2]), ([100, n - 100, 0], [1, 0, 2])):
-                want = ref_stream_ops(ref, d, q, w, sizes, ops)
+                want = ref.stream_ops(d, q, w, sizes, ops)
                 pos, cuts, acc, fixed, hint = 0, [], 0, False, 0
                 for a, op in zip(sizes, ops):
                     if not fixed and (op != 0 or acc + a >= bs):   # encode.c:1619: the size hint freezes at the first EncodeData
@@ -469,7 +463,7 @@ def test_sim_q234_flush_cuts(sim):
                 assert got == want, (q, w, sizes, ops)
     d = synth_text(4 * 65536, 9)
     for q, w in ((2, 22), (3, 22), (4, 22)):
-        want = ref_stream_ops(ref, d, q, w, [len(d), 0], [0, 2])          # FINISH without input behind full blocks
+        want = ref.stream_ops(d, q, w, [len(d), 0], [0, 2])          # FINISH without input behind full blocks
         assert _sim_cuts(sim, d, q, w, 1 << (14 if q < 4 else 16), [], [], 1, finish_empty=1) == want, (q, w)
 
 
@@ -568,19 +562,17 @@ def test_sim_flush_just_behind_a_block_boundary(sim):
     (hash_longest_match_quickly_inc.h:119 / hash_longest_match64_inc.h:127: num_bytes >= HashTypeLength - 1); the block behind
     it stitches instead, and its three positions reach back across the short block into the block in front.  Their owner must
     still commit them (br_commit_bits; found by a randomized FLUSH campaign: q3, lgwin 12, flush at 14 * 16384 + 2)."""
-    from brotli_libs import REF_SO, Ref, ref_stream_ops
-    if not os.path.exists(REF_SO):
-        pytest.skip("oracle/_ref not built")
+    from brotli_libs import RecordedRef
     from corpus import synth_text
-    ref = Ref()
+    ref = RecordedRef()
     d = synth_text(200000, 77)
     n = len(d)
     for q, w in ((3, 12), (2, 22), (4, 16), (5, 22), (7, 17)):
         bs = 1 << (14 if q < 4 else 16)
         for extra in (1, 2, 3, 5, 6):
             c = 2 * bs + extra
-            want = ref_stream_ops(ref, d, q, w, [c, n - c], [1, 2])
+            want = ref.stream_ops(d, q, w, [c, n - c], [1, 2])
             assert _sim_cuts(sim, d, q, w, c, [c], [1], 1) == want, (q, w, extra)
         c1, c2 = bs + 1, bs + 2                                    # two short blocks in a row
-        want = ref_stream_ops(ref, d, q, w, [c1, 1, n - c2], [1, 1, 2])
+        want = ref.stream_ops(d, q, w, [c1, 1, n - c2], [1, 1, 2])
         assert _sim_cuts(sim, d, q, w, c1, [c1, c2], [1, 1], 1) == want, (q, w)

@@ -1,8 +1,8 @@
 """GPU suite (-m gpu), last file on purpose: qualities 2..4 (SURVEY.md 8f rank 1 -- the one-position-per-slot hashers
 H2 / H3 / H4 / H54 of c/enc/hash_longest_match_quickly_inc.h, BrotliStoreMetaBlockFast / Trivial of
-c/enc/brotli_bit_stream.c:1196-1317) through the C ABI, against digests of the compiled reference, the oracle and --
-where it travelled -- oracle/_ref itself.  Bit-exact.  The device functions of this path are the ones tests/test_sim.py
-runs on the CPU (test_sim_q234_*); what only these tests cover is the CUDA plumbing around them: the 32-bit three-pass
+c/enc/brotli_bit_stream.c:1196-1317) through the C ABI, against digests of the compiled reference, the oracle and the
+reference's recorded outputs (brotli_libs.RecordedRef).  Bit-exact.  The device functions of this path are the ones
+tests/test_sim.py runs on the CPU (test_sim_q234_*); what only these tests cover is the CUDA plumbing around them: the 32-bit three-pass
 radix sort of the slot keys, k_walk<0>, k_verify, k_prep_flat and the host wrapper."""
 import ctypes as C
 import hashlib
@@ -12,7 +12,7 @@ import os
 import numpy as np
 import pytest
 
-from brotli_libs import REF_SO, Oracle, Ref, ref_stream_ops
+from brotli_libs import Oracle, RecordedRef
 from golden_cases import make_case
 
 pytestmark = [pytest.mark.gpu, pytest.mark.timeout(900)]
@@ -33,6 +33,8 @@ def _same(got, want, ctx):
     """Byte equality with a useful failure message (this is the path's first run on hardware)."""
     if got == want:
         return
+    if not isinstance(want, bytes):
+        raise AssertionError("%r: %d bytes against %r" % (ctx, len(got), want))
     k = next((i for i in range(min(len(got), len(want))) if got[i] != want[i]), min(len(got), len(want)))
     raise AssertionError("%r: %d bytes against %d, first difference at byte %d" % (ctx, len(got), len(want), k))
 
@@ -118,12 +120,11 @@ def _drive(b200, d, q, w, sizes, ops):
     return out
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_q234_streaming_flush_and_metadata(b200):
     """PROCESS / FLUSH / EMIT_METADATA / FINISH at quality 2..4 (input blocks of 1 << 14 bytes below quality 4), byte-identical
     to the reference's CompressStream for the same call sequence."""
     from corpus import synth_binary, synth_text
-    ref = Ref()
+    ref = RecordedRef()
     for d in (synth_text(500000, 61), synth_binary(600000, 62)):
         n = len(d)
         for q, w in ((2, 22), (3, 16), (4, 22), (4, 11)):
@@ -137,7 +138,7 @@ def test_q234_streaming_flush_and_metadata(b200):
                 ([0, 100, 0, 0, 11, n - 111], [3, 1, 3, 1, 3, 2]),
             ]
             for sizes, ops in seqs:
-                want = ref_stream_ops(ref, d, q, w, sizes, ops)
+                want = ref.stream_ops(d, q, w, sizes, ops)
                 got = _drive(b200, d, q, w, sizes, ops)
                 assert got == want, (q, w, sizes, ops, len(got), len(want))
 
@@ -165,12 +166,11 @@ def test_q234_batch_api(b200):
         assert got == [ora.compress(s, q, 22) for s in many], q
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_q234_full_size(b200):
     """100 MB of text (BASELINE config C2's input) at quality 2 and 4, and 64 MiB of the binary mix at quality 3 with a 24-bit
-    window, against the reference itself on the box."""
+    window, against the reference's recorded outputs."""
     from corpus import synth_binary, synth_text
-    ref = Ref()
+    ref = RecordedRef()
     d = synth_text(100_000_000, 20250922)
     for q in (2, 4):
         _same(b200.compress_oneshot(d, q, 22), ref.compress(d, q, 22), q)
@@ -241,19 +241,18 @@ def test_batch_device_resident_quality_2_to_9(b200):
                 assert out_off[cnt] == sum(len(x) for x in want)
 
 
-@pytest.mark.skipif(not os.path.exists(REF_SO), reason="oracle/_ref did not travel")
 def test_flush_just_behind_a_block_boundary(b200):
     """All qualities: a FLUSH one or two bytes behind a block boundary leaves a block too short to stitch; the positions the
     block behind it stitches reach back across it (tests/test_sim.py::test_sim_flush_just_behind_a_block_boundary: the case a
     randomized campaign found in the last session, wrong bytes before the fix of br_commit_bits)."""
     from corpus import synth_text
-    ref = Ref()
+    ref = RecordedRef()
     d = synth_text(300000, 77)
     n = len(d)
     for q, w in ((3, 12), (2, 22), (4, 16), (5, 22), (7, 17), (9, 24)):
         bs = 1 << (14 if q < 4 else 18 if q >= 9 else 16)
         for extra in (1, 2, 3, 6):
             c = bs + extra
-            _same(_drive(b200, d, q, w, [c, n - c], [1, 2]), ref_stream_ops(ref, d, q, w, [c, n - c], [1, 2]), (q, w, extra))
+            _same(_drive(b200, d, q, w, [c, n - c], [1, 2]), ref.stream_ops(d, q, w, [c, n - c], [1, 2]), (q, w, extra))
         c1, c2 = bs + 1, bs + 2
-        _same(_drive(b200, d, q, w, [c1, 1, n - c2], [1, 1, 2]), ref_stream_ops(ref, d, q, w, [c1, 1, n - c2], [1, 1, 2]), (q, w, "two short blocks"))
+        _same(_drive(b200, d, q, w, [c1, 1, n - c2], [1, 1, 2]), ref.stream_ops(d, q, w, [c1, 1, n - c2], [1, 1, 2]), (q, w, "two short blocks"))
